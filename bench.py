@@ -90,6 +90,33 @@ def synthetic_state_dict(cfg: dict, device, seed: int = 0):
     return sd
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 19              # elements kept of a supplementary output (2 MB): the headline output is written whole
+DUMP_SAMPLE_ONE = 1 << 22          # elements kept of the one output of a --workload vae* run (16 MB of a 0.9 - 1 GB video)
+
+
+def dump_sample(t: torch.Tensor, n: int = DUMP_SAMPLE) -> torch.Tensor:
+    """`t` flattened, or a fixed sample of n of its elements when it has more: the positions are drawn from a seeded generator
+    and depend only on t.numel(), so two runs of the same workload sample the same elements."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= n:
+        return flat.float().cpu()
+    idx = torch.randint(flat.numel(), (n,), generator=torch.Generator().manual_seed(0)).sort().values
+    return flat[idx.to(flat.device)].float().cpu()
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """Write every output as <out_dir>/<name>.npy in float32 (at most DUMP_LIMIT_BYTES in all)."""
+    import numpy as np
+    arrays = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"outputs to dump are {total} bytes, more than {DUMP_LIMIT_BYTES}"
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def measured_peaks():
     f = ROOT / "MEASURED_PEAKS.json"
     if f.exists():
@@ -268,10 +295,11 @@ def _timed_simple(fn, steps, warmup, dev_index=0):
     return ms, clocks.summary(), ops.launch_count() // steps, ops.flop_count() / steps / 1e12, out
 
 
-def supplementary(args, dev, eng5, world, rank, peaks):
-    """The other BASELINE.json configs, run AFTER the headline so the driver's record holds them too (each with its own
+def supplementary(args, dev, eng5, world, rank, peaks, dumps=None):
+    """The other BASELINE.json configs, run AFTER the headline so the bench line holds them too (each with its own
     clocks and roofline): configs[3] 5B 4-step distilled loop (+SDE), a 14B FramePack-chunk forward and a 5-step slice of
-    configs[2] (50-step ODE with CFG), and at N = 1 the three VAE decodes (configs[4] hyvideo; Wan2.2 / Wan2.1)."""
+    configs[2] (50-step ODE with CFG), and at N = 1 the three VAE decodes (configs[4] hyvideo; Wan2.2 / Wan2.1).
+    With `dumps`, rank 0 stores there a sample (dump_sample) of each entry's result from its last timed repetition."""
     import torch.distributed as dist
 
     from yume_b200 import ops, sampler
@@ -298,6 +326,8 @@ def supplementary(args, dev, eng5, world, rank, peaks):
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         ms = float(ms)
+        if dumps is not None and rank == 0:
+            dumps[name] = dump_sample(res)
         tf = flops_per_fwd * fwd_per_loop / (ms * 1e-3) / 1e12
         out[name] = {"ms_per_loop": ms, "forwards_per_loop": fwd_per_loop, "ms_per_forward": ms / fwd_per_loop,
                      "value": new_frames / (ms * 1e-3), "unit": "new latent-frames/s (new_frames / loop time)",
@@ -409,6 +439,8 @@ def supplementary(args, dev, eng5, world, rank, peaks):
 
         def vae_entry(name, eng, z, frames_of, config, encode=False):
             ms, clocks, launches, tflop, res = _timed_simple((lambda: eng.encode(z)) if encode else (lambda: eng.decode(z)), 2, 1, li)
+            if dumps is not None:
+                dumps[name] = dump_sample(res)
             frames = frames_of(res)
             out[name] = {"ms_per_decode": ms, "value": frames / (ms * 1e-3), "unit": ("encoded" if encode else "decoded") + " frames/s",
                          "frames": frames,
@@ -505,17 +537,18 @@ def product_arm(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(total ms of `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     n_warm = args.warmup if args.quick else max(3, args.warmup)
     for _ in range(n_warm):
@@ -525,20 +558,24 @@ def product_arm(args):
     # ---- value: K steps, device-resident inputs, NO per-kernel instrumentation inside the timed region ----
     with ClockSampler(local_rank) as clocks:
         ops.reset_launch_count()
-        total_ms = timed(step_device, args.steps)
+        total_ms, last = timed(step_device, args.steps)
         launches = ops.launch_count()
+    dumps = None
+    if args.dump_outputs and rank == 0:
+        dumps = {"latent_out": last.float().cpu()}                 # the denoised latent [48, 21, 44, 80] of the last timed step
+    del last
     # ---- e2e: the same step through the reference-facing WanModel.forward with pinned HOST tensors ----
     if args.quick:
         e2e_ms = float("nan")
     else:
         for _ in range(2):
             step_e2e()
-        e2e_ms = timed(step_e2e, args.steps)
+        e2e_ms, _ = timed(step_e2e, args.steps)
     # ---- per-kernel table: a SEPARATE instrumented pass (CUDA events around tagged launches on the launching stream) ----
     k_steps = min(args.steps, 5)
     eng.timer.reset()
     eng.timer.active = True
-    instr_ms = timed(step_device, k_steps)
+    instr_ms, _ = timed(step_device, k_steps)
     eng.timer.active = False
     kern = eng.timer.summary()
 
@@ -635,12 +672,14 @@ def product_arm(args):
         holder = {"model": model, "engine": eng}
         del model, eng
         try:
-            sup = supplementary(args, dev, holder, world, rank, peaks)
+            sup = supplementary(args, dev, holder, world, rank, peaks, dumps)
         except Exception as e:
             import traceback
             sup = {"error": f"{type(e).__name__}: {e}", "traceback": traceback.format_exc()[-1500:]}
         if rank == 0:
             line["supplementary"] = sup
+    if dumps is not None:
+        dump_outputs(args.dump_outputs, dumps)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -687,6 +726,8 @@ def chunk_arm(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latent_out": out})
     flops = cfg["num_layers"] * block_flops(L, cfg["dim"], cfg["ffn_dim"], S)
     print(json.dumps({"metric": "latent_frames_per_sec", "value": 8 / (ms * 1e-3), "unit": "latent-frames/s", "n_gpus": 1,
                       "steps": args.steps, "warmup": max(3, args.warmup), "ms_per_step": ms, "higher_is_better": True,
@@ -733,6 +774,8 @@ def vae_arm(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"video": dump_sample(out, DUMP_SAMPLE_ONE)})
     frames = out.shape[2]
     print(json.dumps({"metric": "decoded_frames_per_sec", "value": frames / (ms * 1e-3), "unit": "frames/s", "n_gpus": 1,
                       "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -781,6 +824,8 @@ def vae22_arm(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"video": dump_sample(out, DUMP_SAMPLE_ONE)})
     print(json.dumps({"metric": "decoded_frames_per_sec", "value": out.shape[1] / (ms * 1e-3), "unit": "frames/s", "n_gpus": 1,
                       "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
                       "dtype": "bf16", "data": "synthetic",
@@ -795,7 +840,7 @@ def main():
     ap.add_argument("--config", default="5b-720p", choices=["5b-720p", "5b-chunk", "14b-chunk"],
                     help="5b-720p is the headline workload (BASELINE.json configs[1]); the others are supplementary")
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="yume_b200", choices=["yume_b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -805,7 +850,13 @@ def main():
     ap.add_argument("--sp-transport", default="auto", choices=["auto", "p2p", "p2p_gemm", "nccl"])
     ap.add_argument("--gemm-split-k", type=int, default=0, choices=[0, 1], help="tail split-K of the gate+residual GEMMs: 0 automatic, 1 never (A/B)")
     ap.add_argument("--quick", action="store_true", help="profiling runs: exact --warmup, no e2e leg, no CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32; the headline "
+                         "latent whole, each supplementary result and a VAE video as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    torch.manual_seed(0)     # draws without an explicit generator (the SDE loop's noise) repeat from run to run
     if args.gemm_split_k:
         from yume_b200 import ops as _ops
         _ops.GEMM_SPLIT_K = args.gemm_split_k

@@ -304,22 +304,16 @@ def test_conv_tile_plan():
 
 
 @pytest.mark.parametrize("tree,cfg_name", [("wan23", "CFG_5B_TINY"), ("wan", "CFG_14B_TINY")])
-def test_install_on_the_reference_wanmodel_repacks_identically(tree, cfg_name):
-    """Drop-in boundary (SURVEY.md §8b): `install()` on a live REFERENCE `WanModel` — loaded from /root/reference with the
-    recipe of tools/make_golden.py — must re-bind `forward` and build, from the module's own parameters
-    (`WanDiT.from_module`), exactly the packed tensors the state-dict path builds. Runs where the reference tree exists (the
-    authoring container); skipped on the GPU box."""
-    import sys
-    ref_root = Path("/root/reference")
-    if not (ref_root / tree / "modules" / "model.py").exists():
-        pytest.skip("reference tree not present")
-    sys.path.insert(0, str(ROOT / "tools"))
-    import make_golden
+def test_install_on_the_reference_wanmodel_repacks_identically(golden_dir, tree, cfg_name):
+    """Drop-in boundary (SURVEY.md §8b): `install()` on a live `WanModel` — a module with the parameter layout and attributes
+    recorded from the REFERENCE's own class (tests/helpers/reference_modules.py) — must re-bind `forward` and build, from the
+    module's own parameters (`WanDiT.from_module`), exactly the packed tensors the state-dict path builds."""
+    from helpers import reference_modules
     from yume_b200 import model as ybm
     cfg = getattr(synth, cfg_name)
     sd = synth.make_state_dict(cfg, 4321)
-    ref_model = make_golden.build_reference_model(make_golden.load_reference(tree), cfg, sd)
-    assert type(ref_model).__module__.startswith(tree)                 # really the reference's class
+    rec = torch.load(golden_dir / "install_dit.pt", weights_only=False)[cfg_name]
+    ref_model = reference_modules.wanmodel(cfg, sd, rec)
     ref_forward = ref_model.forward
     ybm.install(ref_model, device="cpu")                               # repack only: no kernel runs at install time
     assert ref_model.forward is not ref_forward and ref_model.forward.__func__ in (ybm.forward_5b, ybm.forward_14b)

@@ -1,20 +1,17 @@
-"""Drop-in hooks of the Wan VAEs on the REFERENCE's own classes, on CPU: build `WanVAE_` from /root/reference (2.2 and 2.1 trees) with
-seeded weights, wrap it the way `Wan2_2_VAE` / `WanVAE` hold it (`.model`, `.scale` / `.mean`, `.std`; their constructors want a
-checkpoint file), run the reference's own chunked encode / decode, then `install_*` on the wrapper and call `encode(list)` /
-`decode(list)` — list in / list out, outputs within the bf16 budget of the reference's fp32 result. The engines run over the torch
-stand-in for the C ABI (tests/helpers/torch_ops.py). Authoring container only (skipped where /root/reference is absent)."""
-import importlib.util
+"""Drop-in hooks of the Wan VAEs and the hyvideo VAE on CPU: `install_*` on a wrapper holding a module with the parameter layout and the
+attributes of the REFERENCE's own class (`WanVAE_` of the 2.2 and 2.1 trees, `AutoencoderKLCausal3D`; tests/helpers/reference_modules.py),
+held the way `Wan2_2_VAE` / `WanVAE` hold it (`.model`, `.scale` / `.mean`, `.std`; their constructors want a checkpoint file), then
+`encode(list)` / `decode(list)` — list in / list out, outputs within the bf16 budget of what the reference's own chunked encode / decode
+computed from the same seeded weights and inputs (tests/golden/install_vae.pt, tools/make_golden_install.py). The engines run over the
+torch stand-in for the C ABI (tests/helpers/torch_ops.py)."""
 import types
-from pathlib import Path
 
 import pytest
 import torch
 
-from helpers import torch_ops
+from helpers import reference_modules, torch_ops
 from oracle import wan21vae, wan21vae_enc, wan22vae, wan22vae_enc
 from yume_b200 import vae21, vae22, vae_enc
-
-REF = Path("/root/reference")
 
 
 @pytest.fixture()
@@ -23,13 +20,9 @@ def cpu_ops(monkeypatch):
         monkeypatch.setattr(mod, "ops", torch_ops)
 
 
-def _load(path, name):
-    if not path.exists():
-        pytest.skip("reference tree not present")
-    spec = importlib.util.spec_from_file_location(name, str(path))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+@pytest.fixture(scope="module")
+def recorded(golden_dir):
+    return torch.load(golden_dir / "install_vae.pt", weights_only=False)
 
 
 def _rel(a, b):
@@ -37,21 +30,19 @@ def _rel(a, b):
 
 
 @torch.no_grad()
-def test_wan22_wrapper_hooks_are_drop_ins(cpu_ops):
-    ref = _load(REF / "wan23" / "modules" / "vae2_2.py", "ref_vae2_2_install")
+def test_wan22_wrapper_hooks_are_drop_ins(cpu_ops, recorded):
+    rec = recorded["wan22"]
     cfg = dict(dim=32, z_dim=16, dim_mult=(1, 2, 4, 4), num_res_blocks=2, temperal_downsample=(False, True, True))
     sd = dict(wan22vae_enc.make_state_dict(11, **cfg))
     sd.update(wan22vae.make_state_dict(12, dec_dim=32, z_dim=16, dim_mult=(1, 2, 4, 4), num_res_blocks=2, temperal_upsample=(True, True, False)))
-    model = ref.WanVAE_(dim=32, dec_dim=32, z_dim=16, dim_mult=[1, 2, 4, 4], num_res_blocks=2, attn_scales=[],
-                        temperal_downsample=[False, True, True]).eval()
-    model.load_state_dict(sd, strict=True)
+    model = reference_modules.module(sd, rec, dim=32, z_dim=16, dim_mult=[1, 2, 4, 4], num_res_blocks=2,
+                                     temperal_downsample=[False, True, True], temperal_upsample=[True, True, False])
     g = torch.Generator().manual_seed(3)
     mean, std = 0.3 * torch.randn(16, generator=g), 0.5 + torch.rand(16, generator=g)
     wrapper = types.SimpleNamespace(model=model, scale=[mean, 1.0 / std], dtype=torch.float)
     video = torch.randn(3, 5, 32, 64, generator=g).clamp_(-1, 1)
     z = torch.randn(16, 2, 2, 4, generator=g)
-    want_mu = model.encode(video.unsqueeze(0), wrapper.scale).float().squeeze(0)
-    want_x = model.decode(z.unsqueeze(0), wrapper.scale).float().clamp_(-1, 1).squeeze(0)
+    want_mu, want_x = rec["want_mu"], rec["want_x"]
     vae_enc.install_wan22_vae_encoder(wrapper, device="cpu")
     vae22.install_wan22_vae(wrapper, device="cpu")
     got_mu, got_x = wrapper.encode([video]), wrapper.decode([z])
@@ -62,20 +53,19 @@ def test_wan22_wrapper_hooks_are_drop_ins(cpu_ops):
 
 
 @torch.no_grad()
-def test_wan21_wrapper_hooks_are_drop_ins(cpu_ops):
-    ref = _load(REF / "wan" / "modules" / "vae.py", "ref_vae_install")
+def test_wan21_wrapper_hooks_are_drop_ins(cpu_ops, recorded):
+    rec = recorded["wan21"]
     cfg = dict(dim=32, z_dim=16, dim_mult=(1, 2, 4, 4), num_res_blocks=2)
     sd = dict(wan21vae_enc.make_state_dict(21, temperal_downsample=(False, True, True), **cfg))
     sd.update(wan21vae.make_state_dict(22, temperal_upsample=(True, True, False), **cfg))
-    model = ref.WanVAE_(dim=32, z_dim=16, dim_mult=[1, 2, 4, 4], num_res_blocks=2, attn_scales=[], temperal_downsample=[False, True, True]).eval()
-    model.load_state_dict(sd, strict=True)
+    model = reference_modules.module(sd, rec, dim=32, z_dim=16, dim_mult=[1, 2, 4, 4], num_res_blocks=2,
+                                     temperal_downsample=[False, True, True], temperal_upsample=[True, True, False])
     g = torch.Generator().manual_seed(4)
     mean, std = 0.3 * torch.randn(16, generator=g), 0.5 + torch.rand(16, generator=g)
     wrapper = types.SimpleNamespace(model=model, mean=mean, std=std, scale=[mean, 1.0 / std], dtype=torch.float)
     video = torch.randn(3, 5, 16, 32, generator=g).clamp_(-1, 1)
     z = torch.randn(16, 2, 2, 4, generator=g)
-    want_mu = model.encode(video.unsqueeze(0), wrapper.scale).float().squeeze(0)
-    want_x = model.decode(z.unsqueeze(0), wrapper.scale).float().clamp_(-1, 1).squeeze(0)
+    want_mu, want_x = rec["want_mu"], rec["want_x"]
     vae_enc.install_wan21_vae_encoder(wrapper, device="cpu")
     vae21.install_wan21_vae(wrapper, device="cpu")
     got_mu, got_x = wrapper.encode([video]), wrapper.decode([z])
@@ -84,36 +74,31 @@ def test_wan21_wrapper_hooks_are_drop_ins(cpu_ops):
 
 
 @torch.no_grad()
-def test_hyvideo_install_vae_is_a_drop_in(monkeypatch):
-    """`install_vae` on the reference's own `AutoencoderKLCausal3D` (hyvideo/vae/autoencoder_kl_causal_3d.py, loaded with the diffusers
-    stubs of tools/make_golden_vae.py): the module's own tiled decode, then the re-bound `decode(z, return_dict=...)` — same return
-    convention, `enable_tiling()` honoured, output within the bf16 budget."""
-    import sys
-    if not (REF / "hyvideo" / "vae" / "autoencoder_kl_causal_3d.py").exists():
-        pytest.skip("reference tree not present")
-    root = Path(__file__).resolve().parents[1]
-    sys.path.insert(0, str(root / "tools"))
-    import make_golden_vae
+def test_hyvideo_install_vae_is_a_drop_in(monkeypatch, recorded):
+    """`install_vae` on an `AutoencoderKLCausal3D` (the reference's config and decoder layout, its `enable_tiling()` /
+    `disable_tiling()` switch values as recorded): the re-bound `decode(z, return_dict=...)` — same return convention, tiling
+    honoured, output within the bf16 budget of the module's own tiled decode."""
     from oracle import hyvae
     from yume_b200 import vae as ybvae
     monkeypatch.setattr(ybvae, "ops", torch_ops)
-    ak = make_golden_vae.load_reference_vae()
-    cfg = make_golden_vae.TINY
+    rec = recorded["hyvae"]
+    cfg = dict(block_out_channels=(64, 64, 128, 128), layers_per_block=2, latent_channels=16, out_channels=3)
     sd = hyvae.make_state_dict(99, **cfg)
-    ref = ak.AutoencoderKLCausal3D(in_channels=3, out_channels=3, down_block_types=("DownEncoderBlockCausal3D",) * 4,
-                                   up_block_types=("UpDecoderBlockCausal3D",) * 4, block_out_channels=cfg["block_out_channels"],
-                                   layers_per_block=2, act_fn="silu", latent_channels=16, norm_num_groups=32, sample_size=64,
-                                   sample_tsize=16, time_compression_ratio=4, spatial_compression_ratio=8, mid_block_add_attention=True)
-    ref.load_state_dict(sd, strict=False)
-    ref.eval()
-    ref.enable_tiling()
+    ref = reference_modules.module(sd, rec)
+    ref.config = types.SimpleNamespace(norm_num_groups=32, sample_size=64, sample_tsize=16, **cfg)
+    assert {k: reference_modules.plain(getattr(ref.config, k)) for k in rec["config"]} == rec["config"]
+    ref.use_spatial_tiling, ref.use_temporal_tiling = rec["tiling_on"]           # enable_tiling()
     z = torch.randn(1, 16, 6, 10, 12, generator=torch.Generator().manual_seed(5))
-    want = ref.decode(z, return_dict=False)[0]
     ybvae.install_vae(ref, device="cpu")
+
+    def check(dec):
+        assert tuple(dec.shape) == rec["shape"]
+        for key, got in (("sample", dec[..., ::4, ::4]), ("rowsum", dec.sum(-1)), ("colsum", dec.sum(-2))):
+            assert _rel(got, rec[key]) < 3e-2, key
     got = ref.decode(z, return_dict=False)
-    assert isinstance(got, tuple) and got[0].shape == want.shape and _rel(got[0], want) < 3e-2
-    out = ref.decode(z)
-    assert _rel(out.sample, want) < 3e-2
-    ref.disable_tiling()                                          # the hook follows the module's own switches
+    assert isinstance(got, tuple)
+    check(got[0])
+    check(ref.decode(z).sample)
+    ref.use_spatial_tiling, ref.use_temporal_tiling = rec["tiling_off"]          # disable_tiling(): the hook follows the module's switches
     small = torch.randn(1, 16, 2, 4, 6, generator=torch.Generator().manual_seed(6))
-    assert ref.decode(small, return_dict=False)[0].shape == (1, 3, 5, 32, 48)
+    assert ref.decode(small, return_dict=False)[0].shape == rec["small_shape"] == (1, 3, 5, 32, 48)

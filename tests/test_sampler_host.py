@@ -1,32 +1,20 @@
-"""yume_b200/sampler.py against the reference's own code, on CPU: the sigma schedule is compared with `get_sampling_sigmas` EXTRACTED
-from fastvideo/sample/sample_5b.py (AST: the script itself cannot be imported), the SDE update with the statements of
-sample_tts.py:726-744 restated verbatim, and the Euler / CFG loops with an explicit unrolled restatement of sample_5b.py:941-1034 and
-sample.py:755-790 over a toy `transformer`. Reference-reading parts run in the authoring container only."""
-import ast
+"""yume_b200/sampler.py against the reference's own code, on CPU: the sigma schedule is compared with what `get_sampling_sigmas`,
+EXTRACTED from fastvideo/sample/sample_5b.py, returned (tests/golden/sampling_sigmas.json, tools/make_golden_install.py), the SDE update
+with the statements of sample_tts.py:726-744 restated verbatim, and the Euler / CFG loops with an explicit unrolled restatement of
+sample_5b.py:941-1034 and sample.py:755-790 over a toy `transformer`."""
+import json
 import math
-from pathlib import Path
 
-import pytest
 import torch
 
 from yume_b200 import sampler
 
-REF = Path("/root/reference/fastvideo/sample")
 
-
-def test_sigma_schedule_equals_the_reference_function():
-    src = REF / "sample_5b.py"
-    if not src.exists():
-        pytest.skip("reference tree not present")
-    import numpy as np
-    tree = ast.parse(src.read_text())
-    fn = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "get_sampling_sigmas")
-    ns = {"np": np}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), str(src), "exec"), ns)
-    for steps, shift in ((4, 7.0), (50, 3.0), (50, 5.0), (1, 7.0), (30, 1.0)):
-        want = ns["get_sampling_sigmas"](steps, shift)
+def test_sigma_schedule_equals_the_reference_function(golden_dir):
+    for case in json.loads((golden_dir / "sampling_sigmas.json").read_text()):
+        steps, shift, want = case["steps"], case["shift"], case["sigmas"]
         got = sampler.sampling_sigmas(steps, shift)
-        assert len(got) == steps and max(abs(a - float(b)) for a, b in zip(got, want)) < 1e-12
+        assert len(got) == len(want) == steps and max(abs(a - float(b)) for a, b in zip(got, want)) < 1e-12
 
 
 def test_sde_update_equals_the_reference_statements():
